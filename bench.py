@@ -110,6 +110,31 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_ATOMS = 1 << 18  # 152 bytes each over the five per-atom arrays: 38 MB at most
+
+
+def dump_outputs(out_dir, atom, thermo):
+    """--dump-outputs DIR: the state the timed steps leave to a caller, as float64 .npy files --
+    thermo[8] and, for every atom or (above DUMP_ATOMS atoms) a fixed seeded sample of atom indices in
+    ascending order, position[3][m], velocity[3][m], force[3][m], potential[m], virial[9][m] (GPUMD's
+    per-atom layouts).  Inputs are seeded, so two builds run with the same arguments compare array for
+    array."""
+    import torch
+    n = atom.number_of_atoms
+    idx = np.arange(n)
+    if n > DUMP_ATOMS:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_ATOMS, replace=False))
+    idx = torch.as_tensor(idx, device=atom.position_per_atom.device)
+    out = {"thermo": thermo}
+    for name, rows, t in (("position", 3, atom.position_per_atom), ("velocity", 3, atom.velocity_per_atom),
+                          ("force", 3, atom.force_per_atom), ("potential", 1, atom.potential_per_atom),
+                          ("virial", 9, atom.virial_per_atom)):
+        out[name] = t.view(rows, n).index_select(1, idx).squeeze(0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.double().cpu().numpy())
+
+
 def crystal(cells, workload="pbte"):
     from gpumd_b200.structures import fcc, init_velocities, rocksalt_pbte
     if workload == "lj":  # config C2: fcc argon, a = 5.30 A, 80 K
@@ -359,6 +384,8 @@ def side_bench(args, rank, world, local, torch, dist, engine):
     ms = float(ms_t.item())
     check()
     th = get_thermo()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, atom, thermo)
     stage_ms = None
     if world == 1 and hasattr(pot, "profile"):
         pot.profile(True)
@@ -593,6 +620,8 @@ def ours(args, rank, world):
         ms = float(t.item())
     value = n * world * args.steps / (ms * 1e-3)
     t_final = thermo.cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, atom, thermo)
 
     if rank != 0:
         if world > 1:
@@ -734,9 +763,13 @@ def main():
                     help="skip the run of oracle/_ref/gpumd_ref (the reference on the same GPU) after the bench")
     ap.add_argument("--workload", default="pbte", choices=["pbte", "lj", "unep", "si"],
                     help="pbte = the BASELINE metric (C3); lj / unep / si = secondary lines for C2 / C4 / C5")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the state they computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        raise SystemExit("bench.py: --dump-outputs is for single-GPU runs of --impl ours")
     if args.impl == "reference":
         reference_arm(args, rank, world)
     else:

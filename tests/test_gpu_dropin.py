@@ -37,7 +37,7 @@ def run(tmp, b200, timeout=900):
 @pytest.fixture(scope="module")
 def exe():
     if not EXE.exists():
-        pytest.skip("oracle/_ref/gpumd_b200 not built (make -C oracle -f Makefile.gpumd_b200; needs /root/reference)")
+        pytest.skip("oracle/_ref/gpumd_b200 not built (build() with GPUMD_REFERENCE naming a GPUMD source tree)")
     return EXE
 
 

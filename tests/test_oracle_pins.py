@@ -52,22 +52,13 @@ def test_bazro3_golden_regression(oracle, precision):
     ("nep_PbTe_static.txt", "static"), ("nep_BaZrO3.txt", "bazro3"), ("nep_PbTe.txt", "c1"),
     ("nep_synth_50types.txt", "synth50")])
 def test_oracle_matches_reference_nep_cpu(oracle, model, structure):
-    """FP64 restatement vs the reference's own NEP_CPU compiled from /root/reference (oracle/_ref).
+    """FP64 restatement vs the reference's own NEP_CPU (tests/golden/refcpu_nep.npz: its energies,
+    forces and virials with the inputs they were computed on; tests/golden/make_fixtures.py).
     Differences come only from NEP_CPU keeping the parameters in double while the GPU reference
     (and the restatement) round them to float on load."""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/libnep_cpu_ref.so not built")
-    order = nep_type_order(GOLDEN / model)
-    if structure == "static":
-        s = read_xyz(GOLDEN / "gpumd_static_model.xyz", order)
-    elif structure == "bazro3":
-        s = read_xyz(GOLDEN / "BaZrO3-nat40-rattled.xyz", order)
-    elif structure == "synth50":  # 50 random species (tests/golden/make_synthetic_models.py)
-        from cases import NEP_CASES_SYNTH
-        s = NEP_CASES_SYNTH["synth50"][1]()
-    else:  # config C1: 216-atom rocksalt PbTe, rattle 0.05 A, seed 1
-        s = rocksalt_pbte(3, rattle=0.05, seed=1)
-    ref = oracle.RefNepCpu(GOLDEN / model).compute(s["type"], s["h"], s["pos"])
+    d = np.load(GOLDEN / "refcpu_nep.npz")
+    s = {k: d[f"{structure}_{k}"] for k in ("type", "h", "pbc", "pos")}
+    ref = {k: d[f"{structure}_{k}"] for k in ("pe", "force", "virial")}
     r = oracle.NepOracle(GOLDEN / model).compute(s["type"], s["h"], s["pbc"], s["pos"], precision=64)
     n = s["type"].shape[0]
     assert abs(r["pe"].sum() - ref["pe"].sum()) / n < 1e-7
